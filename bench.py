@@ -2,7 +2,7 @@
 """bench.py -- rays/s of the FruitNeRF hot path (fused field + compositing, forward + backward) on
 synthetic 4096-ray x 192-sample batches (BASELINE.json metric), N GPUs of one node.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--variant small|big] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--variant small|big] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch: render forward (hash encode -> MLPs ->
 composite), MSE + BCE loss, backward into the flat gradient buffer (and, for N > 1, one NCCL
@@ -140,6 +140,36 @@ def _ncu_traffic(kernel: str):
     return (j["dram_bytes"], j["capture"]) if j else (None, None)
 
 
+DUMP_MAX_BYTES = 64_000_000
+DUMP_SAMPLE_ELEMS = 1 << 20
+
+
+def dump_outputs(step, field, out_dir: str) -> None:
+    """Write what the last timed step handed its caller -- the loss, the render outputs and the parameter gradients -- as
+    ``out_dir/<name>.npy`` (float32), so that two builds run with the same arguments can be compared array by array.  A gradient
+    of more than DUMP_SAMPLE_ELEMS elements (the hash table's) is written as a sample of its rows drawn with a fixed seed, so
+    every run writes the same rows."""
+    import numpy as np
+
+    names = {id(p): n for n, p in field.named_parameters()}
+    arrays = {"loss": step.loss, **{f"out.{k}": v for k, v in step.outputs.items()}}
+    for p in step.params:
+        g = p.grad
+        if g.numel() > DUMP_SAMPLE_ELEMS:
+            n_rows = DUMP_SAMPLE_ELEMS * g.shape[0] // g.numel()
+            rows = torch.randint(0, g.shape[0], (n_rows,), generator=torch.Generator().manual_seed(0)).unique()
+            g = g[rows.to(g.device)]
+        arrays[f"grad.{names[id(p)]}"] = g
+    host = {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+    total = sum(a.nbytes for a in host.values())
+    if total > DUMP_MAX_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_MAX_BYTES}-byte limit")
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    for k, a in host.items():
+        np.save(out / f"{k}.npy", a)
+
+
 def kernel_names(variant: str, kernel: str):
     if kernel == "simt":
         return "simt_field_forward_kernel + simt_composite_kernel", "simt_field_backward_kernel"
@@ -153,8 +183,10 @@ def _stage(msg: str) -> None:
         print(f"[bench {time.strftime('%H:%M:%S')}] {msg}", file=sys.stderr, flush=True)
 
 
-def measure_variant(variant: str, steps: int, warmup: int, args, world: int, rank: int, dev, impl_id, with_e2e: bool = True):
-    """Device-timed step / forward / backward and (optionally) the end-to-end loop of one field variant."""
+def measure_variant(variant: str, steps: int, warmup: int, args, world: int, rank: int, dev, impl_id, with_e2e: bool = True,
+                    dump_dir=None):
+    """Device-timed step / forward / backward and (optionally) the end-to-end loop of one field variant; with ``dump_dir``,
+    rank 0 writes the outputs of the last timed step there (dump_outputs)."""
     from fruitnerf_b200 import _lib as L
     from fruitnerf_b200 import ops
     from fruitnerf_b200 import synthetic as syn
@@ -217,6 +249,8 @@ def measure_variant(variant: str, steps: int, warmup: int, args, world: int, ran
 
         dist.barrier()
     clocks = sampler.stop() if sampler else None
+    if dump_dir is not None and rank == 0:
+        dump_outputs(step, field, dump_dir)
     step_ms = [ev[0].elapsed_time(ev[1]) for ev in evs]
     if os.environ.get("FNR_BENCH_DEBUG"):
         print(f"rank {rank} {variant} step_ms " + " ".join(f"{v:.3f}" for v in step_ms), file=sys.stderr)
@@ -315,12 +349,11 @@ def measure_variant(variant: str, steps: int, warmup: int, args, world: int, ran
     e2e = None
     _stage(f"{variant}: e2e loop")
     if with_e2e:
-        e2e_steps = max(steps, 20)
         torch.cuda.synchronize()
         t0 = time.perf_counter()
         step.load_packed(packed)
         pending, losses = None, []
-        for i in range(e2e_steps):
+        for i in range(steps):
             # H2D of the NEXT step's rays / bins / targets (one packed pinned buffer) overlaps this step, as a prefetching
             # data loader does; the loss of step i is copied device->host asynchronously into pinned memory and read on the host
             # one step later (no per-step drain of the GPU); every step still moves one full batch host->device and one loss
@@ -334,14 +367,14 @@ def measure_variant(variant: str, steps: int, warmup: int, args, world: int, ran
             pending = handle
         losses.append(pending.value())
         torch.cuda.synchronize()
-        assert len(losses) == e2e_steps and all(v == v for v in losses)
+        assert len(losses) == steps and all(v == v for v in losses)
         e2e_s = torch.tensor([time.perf_counter() - t0], device=dev, dtype=torch.float64)
         if world > 1:
             import torch.distributed as dist
 
             dist.all_reduce(e2e_s, op=dist.ReduceOp.MAX)
-        e2e = {"value": world * R_RAYS * e2e_steps / float(e2e_s), "unit": "rays/s", "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": 4,
-               "steps": e2e_steps}
+        e2e = {"value": world * R_RAYS * steps / float(e2e_s), "unit": "rays/s", "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": 4,
+               "steps": steps}
     if world > 1:
         import torch.distributed as dist
 
@@ -474,14 +507,14 @@ def run_ours(args):
         dist.init_process_group("nccl", device_id=dev)
     impl_id = {"auto": L.FNR_IMPL_AUTO, "simt": L.FNR_IMPL_SIMT, "tcgen05": L.FNR_IMPL_TCGEN05}[args.kernel]
     warm = max(args.warmup, 3)
-    head = measure_variant(args.variant, args.steps, warm, args, world, rank, dev, impl_id)
+    head = measure_variant(args.variant, args.steps, warm, args, world, rank, dev, impl_id, dump_dir=args.dump_outputs)
     variants = {}
     if args.variant == "small" and not args.no_variants:
-        # BASELINE.json configs[2] / [3]: fruit_nerf_big, same batch shape, same timing rules (fewer timed steps)
+        # BASELINE.json configs[2] / [3]: fruit_nerf_big, same batch shape, same timing rules
         try:
-            b = measure_variant("big", max(3, min(args.steps, 10)), 3, args, world, rank, dev, impl_id)
+            b = measure_variant("big", args.steps, 3, args, world, rank, dev, impl_id)
             b["config"] = {"workload": f"fruit_nerf_big field: {R_RAYS} rays x {S_SAMPLES} samples per GPU, render fwd + MSE/BCE loss + bwd"
-                                       + (" + gradient exchange" if world > 1 else ""), "steps": max(3, min(args.steps, 10)), "warmup": 3}
+                                       + (" + gradient exchange" if world > 1 else ""), "steps": args.steps, "warmup": 3}
             b.pop("clocks", None)
             variants["big"] = b
         except Exception as ex:  # noqa: BLE001 -- never allowed to break the headline line
@@ -680,7 +713,9 @@ def main():
         faulthandler.dump_traceback_later(int(os.environ.get("FNR_BENCH_WATCHDOG", "60")), exit=False)
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed steps of every hot-path loop (headline, phases, e2e, big variant); the export and "
+                         "whole-training-iteration figures keep their fixed workloads")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--variant", default="small", choices=["small", "big"])
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
@@ -694,7 +729,14 @@ def main():
     ap.add_argument("--no-graph", action="store_true", help="diagnostic: eager step instead of the CUDA-graph step")
     ap.add_argument("--no-flush", action="store_true", help="diagnostic: skip the L2 flush between timed steps")
     ap.add_argument("--no-clocks", action="store_true", help="diagnostic: do not sample nvidia-smi during the timed region")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the loss, render outputs and parameter gradients of the last timed step "
+                         "as DIR/<name>.npy (float32; the hash-table gradient as a fixed, seeded sample of rows)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -141,6 +141,10 @@ def test_model_eval_matches_oracle_pipeline(native_lib, cuda_device):
 
 
 def test_model_train_step_produces_all_gradients(native_lib, cuda_device):
+    # the random initialisation decides whether proposal level 0 gets any interlevel gradient: for some draws its outer bound
+    # already covers every fine weight (loss term and gradient exactly 0, in the oracle too), so the test must not inherit
+    # whatever RNG state the tests before it left behind
+    torch.manual_seed(0)
     cfg = FruitNerfModelConfig(log2_hashmap_size=15, proposal_net_args_list=[
         {"hidden_dim": 16, "log2_hashmap_size": 14, "num_levels": 5, "max_res": 128, "use_linear": False},
         {"hidden_dim": 16, "log2_hashmap_size": 14, "num_levels": 5, "max_res": 256, "use_linear": False}])
